@@ -1,6 +1,6 @@
 """Benchmark of the embedding hot path: embedded chunks/s at 512 tokens (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -22,11 +22,11 @@ Printed JSON (one line, rank 0):
              the measured burst bf16 peak, its DRAM traffic per launch from the committed ncu capture
              (profiles/ncu_traffic.json), and under "whole_step" the step-level achieved TFLOP/s
              (algorithmic matmul FLOPs, SURVEY 8d) against the measured sustained bf16 peak
-  cpu_baseline  the UNMODIFIED reference (baseline/_ref: `distllm.distributed_embedding.embedding_worker`,
+  cpu_baseline  the UNMODIFIED reference (oracle/_ref: `distllm.distributed_embedding.embedding_worker`,
              its own `[timer] [computed-embeddings ...]` reading) on this box's host cores on a bounded
              sample, in a CPU-only subprocess (rank 0, N=1 only); plus the cosine between its embeddings
              and this repository's for the same checkpoint and file.  Falls back to the oracle port
-             (kind "port") when baseline/_ref is absent.
+             (kind "port") when oracle/_ref is absent.
   extra      the other BASELINE configs and the plugin-level numbers, each with its own roofline fraction:
              ragged (lengths ~U{64..512}), c5_esm2_650m (S=1026), c3_mistral7b (B=16, S=4096),
              c4_gather (N > 1: >= 2 M rows per rank through the all-gather), e2e_worker (tokeniser ->
@@ -291,7 +291,7 @@ _CPU_WEIGHTS: dict = {}
 
 
 def cpu_oracle_run(n_chunks: int, batch: int, seed: int = 0):
-    """FALLBACK when baseline/_ref is absent: time the CPU port of the reference path (oracle forward +
+    """FALLBACK when oracle/_ref is absent: time the CPU port of the reference path (oracle forward +
     reference mean pool) on ``n_chunks`` synthetic 512-token chunks.  Returns (seconds, chunks)."""
     from transformers import BertConfig
 
@@ -327,7 +327,7 @@ def run_reference_port(args) -> None:
         'config': {'workload': WORKLOAD, 'global_batch': 8, 'seq_len': SEQ, 'parallelism': 'cpu',
                    'sample_chunks_per_step': per_step},
         'cpu_baseline': {'value': value, 'unit': 'chunks/s', 'cores': threads, 'kind': 'port', 'sample': sample,
-                         'note': 'baseline/_ref absent: the oracle port ran instead of the reference'},
+                         'note': 'oracle/_ref absent: the oracle port ran instead of the reference'},
         'e2e': {'value': value, 'unit': 'chunks/s', 'h2d_bytes_per_step': 0, 'd2h_bytes_per_step': 0},
         'gpu_launches': 0,
     }, args.json_out)
@@ -581,7 +581,7 @@ def cpu_baseline_leg(device) -> dict:
             sec, n = cpu_oracle_run(n_chunks, 8)
             return {'value': n / sec, 'unit': 'chunks/s', 'cores': torch.get_num_threads(), 'kind': 'port',
                     'sample': f'{n} chunks of {SEQ} tokens, batch 8, fp32 torch CPU oracle ({sec:.1f} s); '
-                              'baseline/_ref absent'}
+                              'oracle/_ref absent'}
         ckpt = workloads.write_bert_checkpoint(tmp / 'ckpt')
         sample = workloads.write_token_rows(tmp / 'sample.jsonl', n_chunks, SEQ, BERT_BASE['vocab_size'], seed=123)
         cmd = [sys.executable, str(REPO / 'bench.py'), '--impl', 'reference', '--steps', '1', '--warmup', '0',
@@ -607,6 +607,16 @@ def cpu_baseline_leg(device) -> dict:
                                                'reference on the same HF checkpoint dir and jsonl file '
                                                '(BERT-base shape, 64 chunks x 512 tokens, batch 8, mean pooler)'}
         return base
+
+
+def dump_outputs(out_dir: Path, suffix: str, **arrays: torch.Tensor) -> None:
+    """``--dump-outputs``: what the timed path handed back in its last step, one float32 ``.npy`` per array
+    (1.5 MB per rank), so that two builds can be compared output for output on the same seeded inputs."""
+    import numpy as np
+
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(out_dir / f'{name}{suffix}.npy', t.float().cpu().numpy())
 
 
 def run_native(args) -> None:
@@ -660,12 +670,13 @@ def run_native(args) -> None:
     host = [synthetic_batch(BATCH, SEQ, BERT_BASE['vocab_size'], seed=1000 * rank + i) for i in range(n_distinct)]
     dev = [tuple(t.to(device) for t in b) for b in host]
     pooled = torch.empty((steps * BATCH, hidden), dtype=torch.float32, device=device)
+    last_dist = [None]
 
     def step(i: int) -> None:
         ids, mask, types = dev[i % n_distinct]
         out = pooled[i * BATCH:(i + 1) * BATCH]
         enc.encode_pooled(ids, mask, types, nv.POOL_MEAN_REF, False, out=out)
-        nv.adjacent_cosine_dist(out)
+        last_dist[0] = nv.adjacent_cosine_dist(out)
 
     for i in range(warm):
         step(i % steps)
@@ -689,6 +700,9 @@ def run_native(args) -> None:
     assert gathered.shape[0] == world * steps * BATCH
     del gathered
     value = world * steps * BATCH / elapsed_s
+    if args.dump_outputs:
+        dump_outputs(Path(args.dump_outputs), '' if world == 1 else f'_rank{rank}',
+                     embeddings=pooled[(steps - 1) * BATCH:], adjacent_cosine_dist=last_dist[0])
 
     # ---- end to end through the C-ABI host-buffer call: H2D + compute + D2H inside the timing, and at
     # N > 1 the all-gather of the ranks' results (uploaded again: the user-facing result lives on the host)
@@ -814,7 +828,14 @@ def main() -> None:
     ap.add_argument('--json-out', default=None, help='also write the JSON line to this file')
     ap.add_argument('--embeddings-out', default=None, help='copy the last step embeddings.npy here')
     ap.add_argument('--no-c1', dest='with_c1', action='store_false', help='skip the C1 (1000 x 128-token) run')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help="write the last timed step's pooled embeddings and adjacent-cosine distances to "
+                         'DIR/<name>.npy (native arm)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'native':
+        ap.error('--dump-outputs applies to the native arm')
     # stdout carries exactly one JSON line: everything libraries write to fd 1 while the benchmark
     # runs (NCCL's version banner, progress bars) is sent to stderr; emit() writes to the saved fd
     global _JSON_FD

@@ -1,6 +1,7 @@
-"""Generate tests/golden/*.npz by running the UNMODIFIED reference (``/root/reference``) on CPU.
+"""Generate tests/golden/*.npz by running the UNMODIFIED reference on CPU.
 
-Run in the authoring container only (the reference tree does not exist on the GPU box):
+Needs the reference in ``oracle/_ref``, which ``oracle/ref_shims.install_reference`` copies in first
+(``DISTLLM_REFERENCE=<distllm checkout>`` picks another checkout than its default):
 
     python oracle/make_golden.py
 
@@ -30,7 +31,6 @@ import numpy as np
 import torch
 
 REPO = Path(__file__).resolve().parents[1]
-REFERENCE = Path('/root/reference')
 GOLDEN = REPO / 'tests' / 'golden'
 
 TINY = dict(vocab_size=200, hidden_size=256, num_hidden_layers=2, num_attention_heads=4,
@@ -521,11 +521,13 @@ def make_worker_golden() -> None:
 
 
 def main() -> None:
-    if not REFERENCE.exists():
-        raise SystemExit('/root/reference is not available: golden vectors can only be (re)generated '
-                         'in the authoring container')
-    sys.path.insert(0, str(REFERENCE))
     sys.path.insert(0, str(REPO))
+    from oracle import ref_shims
+
+    print('reference:', ref_shims.install_reference())
+    if ref_shims.reference_root() is None:
+        raise SystemExit('golden vectors are made by the reference: no checkout found, set DISTLLM_REFERENCE')
+    ref_shims.install()
     GOLDEN.mkdir(parents=True, exist_ok=True)
     torch.manual_seed(0)
     make_pool_golden()

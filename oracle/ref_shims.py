@@ -1,11 +1,8 @@
 """Run the UNMODIFIED reference (ramanathanlab/distllm) on CPU.  TEST / BENCH INFRASTRUCTURE ONLY.
 
-The reference is pure Python.  Where it comes from:
-
-  * ``baseline/_ref``   the offline ``pip install --no-deps --target baseline/_ref`` of ``/root/reference``
-                        (git-ignored, travels to the GPU box with the snapshot; made by
-                        ``__graft_entry__.build()`` in the authoring container)
-  * ``/root/reference`` the read-only tree itself (authoring container only)
+The reference is pure Python.  ``install_reference`` copies its ``distllm`` package from an unmodified
+checkout (``$DISTLLM_REFERENCE``, by default ``/root/reference``) into the git-ignored ``oracle/_ref``
+(``__graft_entry__.build()`` does so wherever that checkout exists); everything here imports it from there.
 
 Two of its import-time dependencies are absent from this image and are replaced by the smallest
 stand-ins that let ``distllm.distributed_embedding.embedding_worker`` run (SURVEY 8c):
@@ -25,23 +22,54 @@ from __future__ import annotations
 
 import contextlib
 import io
+import os
 import re
+import shutil
 import sys
+import tempfile
 import types
 from pathlib import Path
 
 REPO = Path(__file__).resolve().parents[1]
-CANDIDATES = (REPO / 'baseline' / '_ref', Path('/root/reference'))
+REF_ROOT = REPO / 'oracle' / '_ref'
+DEFAULT_SOURCE = Path('/root/reference')   # where the unmodified checkout is looked for without $DISTLLM_REFERENCE
 
 _BOUNDARY = re.compile(r'[.!?]["\')\]]*\s+(?=[A-Z0-9"\'(\[])')
 
 
 def reference_root() -> Path | None:
     """Directory to put on ``sys.path`` so that ``import distllm`` finds the unmodified reference."""
-    for root in CANDIDATES:
-        if (root / 'distllm' / 'distributed_embedding.py').exists():
-            return root
+    if (REF_ROOT / 'distllm' / 'distributed_embedding.py').exists():
+        return REF_ROOT
     return None
+
+
+def install_reference() -> str:
+    """Copy the reference's ``distllm`` package from ``$DISTLLM_REFERENCE`` (default ``DEFAULT_SOURCE``) into
+    ``oracle/_ref`` (what ``bench.py --impl reference`` and its ``cpu_baseline`` leg run; without it they time
+    the oracle port).
+    A plain copy is the whole install: the package is pure Python, and its dependency pins (parsl, nltk,
+    bitsandbytes, faiss-gpu ...) are not needed on the embedding path, where the stand-ins below replace
+    the two it imports.  File modes are not copied, so a read-only source gives a removable copy."""
+    if reference_root() is not None:
+        return f'present: {REF_ROOT}'
+    src = os.environ.get('DISTLLM_REFERENCE')
+    pkg = Path(src or DEFAULT_SOURCE) / 'distllm'
+    if not (pkg / 'distributed_embedding.py').exists():
+        if src:
+            raise RuntimeError(f'$DISTLLM_REFERENCE={src} is not a distllm checkout')
+        return f'not installed (no checkout at {DEFAULT_SOURCE}); the CPU arm runs the oracle port'
+    tmp = Path(tempfile.mkdtemp(prefix='_ref.', dir=REF_ROOT.parent))
+    try:
+        shutil.copytree(pkg, tmp / 'distllm', copy_function=shutil.copyfile,
+                        ignore=shutil.ignore_patterns('__pycache__'))
+        for d, _, _ in os.walk(tmp):
+            os.chmod(d, 0o755)
+        shutil.rmtree(REF_ROOT, ignore_errors=True)   # an incomplete earlier copy
+        os.replace(tmp, REF_ROOT)
+    finally:
+        shutil.rmtree(tmp, ignore_errors=True)        # gone already unless the copy failed
+    return f'installed: {REF_ROOT}'
 
 
 def _regex_spans(text: str) -> list[tuple[int, int]]:
@@ -112,7 +140,7 @@ def install(root: Path | None = None) -> Path:
     """Make ``import distllm`` resolve to the unmodified reference; returns the root used."""
     root = root or reference_root()
     if root is None:
-        raise RuntimeError('the reference is not available: neither baseline/_ref nor /root/reference')
+        raise RuntimeError('the reference is not installed in oracle/_ref (see install_reference)')
     if str(root) not in sys.path:
         sys.path.insert(0, str(root))
     _stub_parsl()

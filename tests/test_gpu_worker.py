@@ -3,7 +3,7 @@
 W1 `embedding_worker`, E1 `get_encoder({'name': 'auto' | 'esm2', ...}, register=True)` on local HF checkpoint
 directories (``save_pretrained``), the typer CLI and the torchrun driver -- compared with the outputs the
 UNMODIFIED reference produced for the same checkpoints and texts (tests/golden/*.npz, written by
-oracle/make_golden.py from /root/reference).
+oracle/make_golden.py from the unmodified reference copied into oracle/_ref).
 """
 
 from __future__ import annotations
