@@ -77,7 +77,7 @@ EXPORTS = (
     'b2e_search_ubinary',
     'b2e_layernorm',
 )
-# profiling hooks declared in include/b2e_debug.h (tools/ only; nothing in the package calls them)
+# profiling and test hooks declared in include/b2e_debug.h (tools/ and tests/ only; the package never calls them)
 DEBUG_EXPORTS = (
     'b2e_debug_set_att3_clock',
     'b2e_debug_set_att3_flags',
@@ -87,6 +87,9 @@ DEBUG_EXPORTS = (
     'b2e_debug_set_att3_variant',
     'b2e_debug_set_packing',
     'b2e_debug_topk_tc_fell_back',
+    'b2e_debug_pack_layout',
+    'b2e_debug_gemm_rows',
+    'b2e_debug_attention_packed',
 )
 
 
@@ -347,6 +350,61 @@ def topk_tc_fell_back() -> bool:
     lib.b2e_debug_topk_tc_fell_back.argtypes = [C.POINTER(C.c_int)]
     check(lib.b2e_debug_topk_tc_fell_back(C.byref(out)))
     return bool(out.value)
+
+
+def debug_pack_layout(attention_mask: torch.Tensor, enable: bool = True, storage: str = 'f16'):
+    """Padding-free token layout of a [B, S] int64 mask as the pooled forward pass builds it (debug hook):
+    (cu [B+1], len [B], t_real [2], tok_src [B*S]) int32 CUDA tensors.  tok_src starts as -1; only its first
+    t_real[0] entries are written."""
+    lib = load(storage)
+    _cuda_contig(attention_mask, 'attention_mask')
+    if attention_mask.dtype != torch.int64:
+        raise NativeError('attention_mask must be int64')
+    b, s = attention_mask.shape
+    dev = attention_mask.device
+    cu = torch.full((b + 1,), -1, dtype=torch.int32, device=dev)
+    ln = torch.full((b,), -1, dtype=torch.int32, device=dev)
+    t_real = torch.full((2,), -1, dtype=torch.int32, device=dev)
+    tok_src = torch.full((b * s,), -1, dtype=torch.int32, device=dev)
+    lib.b2e_debug_pack_layout.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int] + [C.c_void_p] * 5
+    with torch.cuda.device(dev):
+        check(lib.b2e_debug_pack_layout(attention_mask.data_ptr(), b, s, int(enable), cu.data_ptr(), ln.data_ptr(),
+                                        t_real.data_ptr(), tok_src.data_ptr(), stream_ptr(dev)), lib)
+    return cu, ln, t_real, tok_src
+
+
+def debug_gemm_rows(a: torch.Tensor, w: torch.Tensor, bias: torch.Tensor | None, resid: torch.Tensor | None,
+                    epilogue: int, m_dev: torch.Tensor, out: torch.Tensor) -> torch.Tensor:
+    """:func:`gemm_h16` into ``out`` with the row count read from the device int32 ``m_dev`` (debug hook): row
+    tiles at or beyond it are left alone."""
+    lib = load(storage_of(a.dtype))
+    for t, what in ((a, 'a'), (w, 'w'), (out, 'out'), (m_dev, 'm_dev')):
+        _cuda_contig(t, what)
+    if m_dev.dtype != torch.int32:
+        raise NativeError('m_dev must be int32')
+    m, k = a.shape
+    n = w.shape[0]
+    lib.b2e_debug_gemm_rows.argtypes = [C.c_void_p] * 5 + [C.c_int] * 4 + [C.c_void_p] * 2
+    with torch.cuda.device(a.device):
+        check(lib.b2e_debug_gemm_rows(a.data_ptr(), w.data_ptr(), _ptr(bias), _ptr(resid), out.data_ptr(), m, n, k,
+                                      epilogue, m_dev.data_ptr(), stream_ptr(a.device)), lib)
+    return out
+
+
+def debug_attention_packed(qkv: torch.Tensor, attention_mask: torch.Tensor, cu: torch.Tensor, seq_len: torch.Tensor,
+                           ctx: torch.Tensor, heads: int, kv_heads: int, head_dim: int, window: int = 0) -> torch.Tensor:
+    """Attention on the packed token layout (debug hook): sequence b in rows cu[b] .. cu[b]+len[b]-1 of ``qkv`` and
+    ``ctx`` (both B*S rows).  head_dim 64: the bidirectional / sliding-window kernel; 128: causal grouped-query."""
+    lib = load(storage_of(qkv.dtype))
+    for t, what in ((qkv, 'qkv'), (attention_mask, 'attention_mask'), (cu, 'cu'), (seq_len, 'len'), (ctx, 'ctx')):
+        _cuda_contig(t, what)
+    b, s = attention_mask.shape
+    lib.b2e_debug_attention_packed.argtypes = [C.c_void_p] * 5 + [C.c_int] * 6 + [C.c_void_p]
+    with torch.cuda.device(qkv.device):
+        check(lib.b2e_debug_attention_packed(qkv.data_ptr(), attention_mask.data_ptr(), cu.data_ptr(),
+                                             seq_len.data_ptr(), ctx.data_ptr(), b, s, heads, kv_heads, head_dim,
+                                             window, stream_ptr(qkv.device)), lib)
+    return ctx
 
 
 def pack_ubinary(embeddings: torch.Tensor) -> torch.Tensor:

@@ -219,9 +219,8 @@ int launch_gemm_bn(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorM
       return launch_gemm_cfg<BN, STAGES, EPI_BIAS>(ta, tb, tout, bias, resid, M, N, K, sms, st, m_dev);
     case B2E_EPI_BIAS_GELU:
       return launch_gemm_cfg<BN, STAGES, EPI_BIAS_GELU>(ta, tb, tout, bias, resid, M, N, K, sms, st, m_dev);
-    case B2E_EPI_BIAS_RESID:
-      return launch_gemm_cfg<BN, STAGES, EPI_BIAS_RESID>(ta, tb, tout, bias, resid, M, N, K, sms,
-                                                         st);
+    case B2E_EPI_BIAS_RESID:   // m_dev used to be dropped here: with N % 256 == 128 every row tile up to M was written
+      return launch_gemm_cfg<BN, STAGES, EPI_BIAS_RESID>(ta, tb, tout, bias, resid, M, N, K, sms, st, m_dev);
     case B2E_EPI_SWIGLU:
       if constexpr (BN == 256)
         return launch_gemm_cfg<256, STAGES, EPI_SWIGLU>(ta, tb, tout, bias, resid, M, N, K, sms, st, m_dev);
@@ -1628,8 +1627,9 @@ int b2e_adjacent_cosine_dist(const void* emb, int dtype, int64_t n_rows, int H,
   return B2E_OK;
 }
 
-int b2e_gemm_h16(const void* A, const void* W, const float* bias, const void* resid, void* out,
-                  int M, int N, int K, int epi, void* stream) {
+// b2e_gemm_h16 and b2e_debug_gemm_rows: m_dev (nullable) = device-resident row count <= M, as in the trunks
+static int gemm_h16_checked(const void* A, const void* W, const float* bias, const void* resid, void* out,
+                            int M, int N, int K, int epi, const int* m_dev, void* stream) {
   if (!A || !W || !out) return fail(B2E_ERR_INVALID, "null tensor pointer");  // bias may be null
   if (epi == B2E_EPI_BIAS_RESID && !resid) return fail(B2E_ERR_INVALID, "resid epilogue needs resid");
   int rc;
@@ -1641,7 +1641,19 @@ int b2e_gemm_h16(const void* A, const void* W, const float* bias, const void* re
   CUtensorMap ta, tb;
   if ((rc = make_tmap_h16(&ta, A, M, K, 128))) return rc;
   if ((rc = make_tmap_h16(&tb, W, N, K, gemm_bn_for(N)))) return rc;
-  return launch_gemm(ta, tb, out, bias, resid, M, N, K, epi, info.sms, (cudaStream_t)stream);
+  return launch_gemm(ta, tb, out, bias, resid, M, N, K, epi, info.sms, (cudaStream_t)stream, m_dev);
+}
+
+int b2e_gemm_h16(const void* A, const void* W, const float* bias, const void* resid, void* out,
+                  int M, int N, int K, int epi, void* stream) {
+  return gemm_h16_checked(A, W, bias, resid, out, M, N, K, epi, nullptr, stream);
+}
+
+// Test hook (b2e_debug.h): b2e_gemm_h16 with the row count read on the device, as the packed trunks run it.
+int b2e_debug_gemm_rows(const void* A, const void* W, const float* bias, const void* resid, void* out,
+                        int M, int N, int K, int epi, const int* m_dev, void* stream) {
+  if (!m_dev) return fail(B2E_ERR_INVALID, "gemm_rows: null device row count");
+  return gemm_h16_checked(A, W, bias, resid, out, M, N, K, epi, m_dev, stream);
 }
 
 int b2e_attention_d64(const void* qkv, const int64_t* mask, void* ctx, int B, int S, int heads,
@@ -1688,6 +1700,53 @@ int b2e_attention_causal_d128(const void* qkv, const int64_t* mask, void* ctx, i
   if ((rc = attention_prepare(g_attn_scratch, mask, B, S, st))) return rc;
   return launch_attention_causal_d128(qkv, g_attn_scratch, ctx, B, S, heads, kv_heads, window,
                                       info.sms, st);
+}
+
+// Test hooks (b2e_debug.h) for the padding-free token layout (pack.cuh): the layout kernels of pack_prepare, and the
+// attention kernels on rows cu[b] .. cu[b] + len[b] - 1 of [B*S]-row buffers, exactly as the encoder runs them.
+int b2e_debug_pack_layout(const int64_t* mask, int B, int S, int enable, int* cu, int* len, int* t_real,
+                          int* tok_src, void* stream) {
+  if (!mask || !cu || !len || !t_real || !tok_src) return fail(B2E_ERR_INVALID, "null tensor pointer");
+  if (B <= 0 || S <= 0) return fail(B2E_ERR_INVALID, "empty batch B=%d S=%d", B, S);
+  int rc;
+  DeviceInfo info;
+  if ((rc = current_device_info(&info))) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  int* scratch = nullptr;   // len_raw | ok, released in stream order
+  CUDA_TRY(cudaMallocAsync(&scratch, sizeof(int) * 2 * (size_t)B, st));
+  pack_lengths_kernel<<<(B + 7) / 8, 256, 0, st>>>(mask, scratch, scratch + B, B, S);
+  pack_scan_kernel<<<1, 256, 0, st>>>(scratch, scratch + B, len, cu, t_real, B, S, enable ? 1 : 0);
+  pack_fill_kernel<<<dim3((S + 255) / 256, B), 256, 0, st>>>(len, cu, tok_src, B, S);
+  const cudaError_t le = cudaGetLastError();
+  CUDA_TRY(cudaFreeAsync(scratch, st));
+  CUDA_TRY(le);
+  return B2E_OK;
+}
+
+int b2e_debug_attention_packed(const void* qkv, const int64_t* mask, const int* cu, const int* len, void* ctx,
+                               int B, int S, int heads, int kv_heads, int head_dim, int window, void* stream) {
+  if (!qkv || !mask || !cu || !len || !ctx) return fail(B2E_ERR_INVALID, "null tensor pointer");
+  if (B <= 0 || S <= 0 || heads <= 0 || window < 0) return fail(B2E_ERR_INVALID, "bad attention problem");
+  if (head_dim == 64 && kv_heads != heads)
+    return fail(B2E_ERR_INVALID, "head_dim 64 attention has no grouped-query form (kv_heads %d != heads %d)",
+                kv_heads, heads);
+  if (head_dim == 128 && (kv_heads <= 0 || heads % kv_heads != 0))
+    return fail(B2E_ERR_INVALID, "heads %d not a multiple of kv_heads %d", heads, kv_heads);
+  if (head_dim != 64 && head_dim != 128) return fail(B2E_ERR_INVALID, "head_dim %d (need 64 or 128)", head_dim);
+  int rc;
+  DeviceInfo info;
+  if ((rc = current_device_info(&info))) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  SeqLayout lay;
+  lay.cu = cu;
+  lay.len = len;
+  if ((rc = attention_prepare(g_attn_scratch, mask, B, S, st))) return rc;
+  if (head_dim == 128)
+    return launch_attention_causal_d128(qkv, g_attn_scratch, ctx, B, S, heads, kv_heads, window, info.sms, st, lay);
+  CUtensorMap tq, tkv;
+  if ((rc = make_tmap_h16(&tq, qkv, (uint64_t)B * S, (uint64_t)3 * heads * AT3_D, 128))) return rc;
+  if ((rc = make_tmap_h16(&tkv, qkv, (uint64_t)B * S, (uint64_t)3 * heads * AT3_D, AT3_KC))) return rc;
+  return launch_attention(tq, tkv, g_attn_scratch, ctx, B, S, heads, info.sms, st, window, lay);
 }
 
 // ---- exact inner-product top-k (retrieval query path)

@@ -3,10 +3,13 @@
  * NOT part of the reference-facing ABI (include/b2e.h): nothing in distllm would bind these.  They
  * exist for the timeline tools under tools/ (att3_timeline.py, gemm_timeline.py, pair_experiments.py)
  * and are declared here so that every symbol the shared library exports is declared in a header.
- * All of them write a __device__ global of the kernels' translation unit; 0 on success.
+ * The set_* hooks write a __device__ global of the kernels' translation unit; the test hooks at the end launch
+ * kernels on caller buffers (tests/).  All return 0 on success.
  */
 #ifndef B2E_DEBUG_H_
 #define B2E_DEBUG_H_
+
+#include <stdint.h>
 
 #ifdef __cplusplus
 extern "C" {
@@ -36,6 +39,24 @@ int b2e_debug_set_att3_variant(int variant);
 int b2e_debug_set_pair_flags(int flags);
 /* device buffer of 4 x 256 int64 filled with clock64() stamps by CTAs 0/1 of the CTA-pair GEMM */
 int b2e_debug_set_clock_buffer(void* device_buffer);
+
+/* Test hooks of the padding-free ("packed") token layout (csrc/pack.cuh), used by tests/.  Pointers are device
+ * pointers; every call is asynchronous on `stream`.
+ *
+ * The layout the pooled forward pass builds from an int64 [B, S] mask: cu [B + 1], len [B], t_real [2] (rows in
+ * use, packed flag) and tok_src [B * S] (only its first t_real[0] entries are written).  enable = 0 forces the
+ * identity layout. */
+int b2e_debug_pack_layout(const int64_t* mask, int B, int S, int enable, int* cu, int* len, int* t_real,
+                          int* tok_src, void* stream);
+/* b2e_gemm_h16 with the row count m_dev (device int, <= M) read on the device: row tiles at or beyond it are
+ * skipped; M sizes the grid and the tensor maps */
+int b2e_debug_gemm_rows(const void* A, const void* W, const float* bias, const void* resid, void* out, int M,
+                        int N, int K, int epi, const int* m_dev, void* stream);
+/* attention on the packed layout: qkv and ctx hold B*S rows, sequence b in rows cu[b] .. cu[b] + len[b] - 1.
+ * head_dim 64: bidirectional (window 0) or sliding-window attention, kv_heads == heads, the variant of
+ * b2e_debug_set_att3_variant; head_dim 128: causal grouped-query attention (window 0 = none). */
+int b2e_debug_attention_packed(const void* qkv, const int64_t* mask, const int* cu, const int* len, void* ctx,
+                               int B, int S, int heads, int kv_heads, int head_dim, int window, void* stream);
 
 #ifdef __cplusplus
 }

@@ -65,6 +65,33 @@ def test_gemm_rejects_bad_shapes(dev, h16):
                      torch.zeros(100, 64, device=dev, dtype=h16), torch.zeros(100, device=dev))
 
 
+@pytest.mark.parametrize('n,epi', [
+    # CTA-pair kernel (N % 256 == 0): every epilogue the trunks use, and the residual one
+    (768, nv.EPI_BIAS), (1024, nv.EPI_BIAS_GELU), (768, nv.EPI_BIAS_RESID), (1536, nv.EPI_SWIGLU),
+    (1536, nv.EPI_GEGLU),
+    # single-CTA kernel (N % 256 == 128; the gated epilogues need N % 256 == 0)
+    (384, nv.EPI_BIAS), (640, nv.EPI_BIAS_GELU), (384, nv.EPI_BIAS_RESID)])
+def test_gemm_device_row_count(dev, n, epi, h16):
+    """The packed trunks pass the row count on the device (t_real): rows below it must equal the plain GEMM bit for
+    bit, row tiles at or beyond it must not be written."""
+    from distllm_b200.embed.encoders.weights import interleave_gate_up
+
+    m_max, k = 20000, 256
+    g = torch.Generator(device=dev).manual_seed(n + epi)
+    a = (torch.randn(m_max, k, device=dev, generator=g) * 0.5).to(h16)
+    w = (torch.randn(n, k, device=dev, generator=g) * 0.08).to(h16)
+    if epi in (nv.EPI_SWIGLU, nv.EPI_GEGLU):
+        w = interleave_gate_up(w[:n // 2], w[n // 2:]).contiguous()
+    bias = torch.randn(n, device=dev, generator=g) * 0.1 if epi <= nv.EPI_BIAS_RESID else None
+    resid = torch.randn(m_max, n, device=dev, generator=g).to(h16) if epi == nv.EPI_BIAS_RESID else None
+    want = nv.gemm_h16(a, w, bias, resid, epi)
+    for m in (1, 127, 128, 129, 255, 256, 257, m_max):
+        out = torch.full_like(want, SENTINEL)
+        nv.debug_gemm_rows(a, w, bias, resid, epi, torch.tensor([m], dtype=torch.int32, device=dev), out)
+        assert torch.equal(out[:m], want[:m]), m
+        assert (out[(m + 255) // 256 * 256:] == SENTINEL).all(), f'rows past m={m} written'
+
+
 @pytest.fixture(params=[None, 5, 0, 69, 64, 193], ids=['shipping', 'two-wg-poly', 'two-wg', 'four-wg-poly', 'four-wg-vote', 'four-wg-epilogue-role'])
 def att_variant(request, h16):
     """Which head_dim-64 attention kernel the calls of a test reach: the library's default (variant 65: four
@@ -81,20 +108,69 @@ def att_variant(request, h16):
     lib.b2e_debug_set_att3_variant(-1)   # back to B2E_ATT3 / the built-in default
 
 
-def ref_attention(qkv, mask, b, s, heads):
-    q, k, v = qkv.float().view(b, s, 3, heads, 64).unbind(2)
-    q, k, v = (t.permute(0, 2, 1, 3) for t in (q, k, v))
-    scores = q @ k.transpose(-1, -2) / 8.0
-    bias = torch.zeros(b, 1, 1, s, device=qkv.device)
-    bias.masked_fill_(mask.view(b, 1, 1, s) == 0, torch.finfo(torch.float32).min)
-    p = torch.softmax(scores + bias, dim=-1)
-    return (p @ v).permute(0, 2, 1, 3).reshape(b * s, heads * 64)
+def ref_attention(qkv, mask, b, s, heads, window=0):
+    """fp32 reference, one sequence at a time (S = 8192 stays in the low GBs); window > 0: |i - j| <= window."""
+    out = torch.empty(b, s, heads * 64, device=qkv.device)
+    i = torch.arange(s, device=qkv.device)
+    band = (i[:, None] - i[None, :]).abs() <= window if window else None
+    for r in range(b):
+        q, k, v = qkv[r * s:(r + 1) * s].float().view(s, 3, heads, 64).permute(1, 2, 0, 3)
+        vis = (mask[r] != 0)[None, :] if band is None else band & (mask[r] != 0)[None, :]
+        scores = (q @ k.transpose(-1, -2) / 8.0).masked_fill_(~vis, torch.finfo(torch.float32).min)
+        out[r] = (torch.softmax(scores, dim=-1) @ v).permute(1, 0, 2).reshape(s, heads * 64)
+        del scores
+    return out.view(b * s, heads * 64)
+
+
+# Rows behind the last packed sequence hold this in K and V (alternating sign), and ctx holds it there before a
+# packed call: a key read past a sequence's length, or a store past its rows, changes the result visibly.  Exact in
+# both 16-bit types.
+SENTINEL = 24576.0
+
+
+def check_packed(qkv, mask, padded_ctx, ref, rows_ok, h16, scale, *, heads, kv_heads=None, head_dim=64, window=0):
+    """The problem `padded_ctx` came from, run again on the library's padding-free token layout
+    (b2e_debug_pack_layout + b2e_debug_attention_packed): rows of the valid tokens must match the fp32 reference
+    (where `rows_ok`) and the padded result bit for bit; rows behind them must stay untouched.  Masks the packer
+    refuses (holes, left padding, empty rows) give the identity layout and the whole padded result."""
+    b, s = mask.shape
+    kv_heads = kv_heads or heads
+    cu, ln, t_real, src = nv.debug_pack_layout(mask, storage=nv.storage_of(h16))
+    t, packed = t_real.tolist()
+    if not packed:
+        assert t == b * s and cu.tolist() == list(range(0, b * s + 1, s)) and ln.tolist() == [s] * b
+        ctx = torch.full_like(padded_ctx, float('nan'))
+        nv.debug_attention_packed(qkv, mask, cu, ln, ctx, heads, kv_heads, head_dim, window)
+        assert torch.equal(ctx, padded_ctx)
+        return
+    src = src[:t].long()
+    qcols = heads * head_dim
+    qkvp = qkv.clone()
+    qkvp[:t] = qkv[src]
+    sign = 1.0 - 2.0 * (torch.arange(qkv.shape[1] - qcols, device=qkv.device) % 2)
+    qkvp[t:, qcols:] = (SENTINEL * sign).to(qkv.dtype)
+    ctx = torch.full_like(padded_ctx, float('nan'))
+    ctx[t:] = SENTINEL
+    nv.debug_attention_packed(qkvp, mask, cu, ln, ctx, heads, kv_heads, head_dim, window)
+    assert torch.isfinite(ctx[:t].float()).all()
+    assert (ctx[t:] == SENTINEL).all(), 'a store landed behind the last sequence'
+    ok = rows_ok[src]
+    close(ctx[:t][ok].float(), ref[src][ok], h16, scale)
+    if head_dim == 128:
+        # Not bit for bit: the causal kernel picks its fast softmax path (one exponential in four as a polynomial)
+        # per warp of 32 query rows, by a vote that also counts the rows behind the sequence's last one -- padding
+        # queries in the padded layout, the next sequence's queries in the packed one (attention4.cuh,
+        # `done = __all_sync(...)`).  Both paths are exact to the storage type: within half its tolerance.
+        close(ctx[:t].float(), padded_ctx[src].float(), h16, 0.5)
+    else:
+        assert torch.equal(ctx[:t], padded_ctx[src]), 'packed and padded layouts differ'
 
 
 @pytest.mark.parametrize('b,s,heads,ragged', [(2, 128, 2, False), (2, 512, 12, False), (3, 200, 12, True),
                                               (2, 512, 12, True), (4, 37, 4, True), (5, 1, 4, False),
                                               (2, 129, 4, True), (1, 384, 12, True), (2, 640, 2, False),
-                                              (1, 1026, 4, True), (3, 257, 2, True)])
+                                              (1, 1026, 4, True), (3, 257, 2, True),
+                                              (8, 1026, 20, True), (2, 8192, 2, True)])
 def test_attention_matches_reference(dev, b, s, heads, ragged, h16, att_variant):
     g = torch.Generator(device=dev).manual_seed(b * 1000 + s)
     qkv = torch.randn(b * s, 3 * heads * 64, device=dev, generator=g).to(h16)
@@ -103,7 +179,42 @@ def test_attention_matches_reference(dev, b, s, heads, ragged, h16, att_variant)
         for i in range(b):
             mask[i, max(1, s - 17 * (i + 1)):] = 0
     ctx = nv.attention_d64(qkv, mask, b, s, heads)
-    close(ctx.float(), ref_attention(qkv, mask, b, s, heads), h16, 2.0)
+    ref = ref_attention(qkv, mask, b, s, heads)
+    close(ctx.float(), ref, h16, 2.0)
+    check_packed(qkv, mask, ctx, ref, mask.bool().view(-1), h16, 2.0, heads=heads)
+
+
+# every edge of the 64-key chunks and 128-row query tiles, mixed in one batch
+EDGE_LENGTHS = [1, 63, 64, 65, 127, 128, 129, 255, 257, 300]
+
+
+@pytest.mark.parametrize('kind', ['full', 'window'])
+def test_attention_packed_length_edges(dev, kind, h16, att_variant):
+    """Sequences of 1 .. S tokens back to back on the packed layout: Q tiles start at arbitrary rows, the last key
+    chunk of every sequence runs into the next one, partial last tiles leave row by row."""
+    attention_length_edges(dev, kind, h16)
+
+
+def test_attention_causal_d128_packed_length_edges(dev, h16):
+    attention_length_edges(dev, 'causal', h16)
+
+
+def attention_length_edges(dev, kind, h16):
+    b, s = len(EDGE_LENGTHS), max(EDGE_LENGTHS)
+    heads, kv_heads, d, window = (6, 6, 64, 0) if kind == 'full' else (4, 4, 64, 64) if kind == 'window' else (4, 2, 128, 100)
+    g = torch.Generator(device=dev).manual_seed(17 + len(kind))
+    qkv = torch.randn(b * s, (heads + 2 * kv_heads) * d, device=dev, generator=g).to(h16)
+    lens = torch.tensor(EDGE_LENGTHS[3:] + EDGE_LENGTHS[:3])   # not sorted: short rows between long ones
+    mask = (torch.arange(s)[None] < lens[:, None]).long().to(dev)
+    if kind == 'causal':
+        ctx = nv.attention_causal_d128(qkv, mask, b, s, heads, kv_heads, window)
+        ref, rows_ok = ref_attention_causal(qkv, mask, b, s, heads, kv_heads, window)
+    else:
+        ctx = nv.attention_d64_window(qkv, mask, b, s, heads, window) if window else nv.attention_d64(qkv, mask, b, s, heads)
+        ref, rows_ok = ref_attention(qkv, mask, b, s, heads, window), torch.ones(b * s, dtype=torch.bool, device=dev)
+    valid = mask.bool().view(-1)
+    close(ctx.float()[valid & rows_ok], ref[valid & rows_ok], h16, 2.0)
+    check_packed(qkv, mask, ctx, ref, rows_ok, h16, 2.0, heads=heads, kv_heads=kv_heads, head_dim=d, window=window)
 
 
 def test_attention_mask_with_holes_and_fully_masked_row(dev, h16, att_variant):
@@ -120,6 +231,12 @@ def test_attention_mask_with_holes_and_fully_masked_row(dev, h16, att_variant):
     ref = ref_attention(qkv, mask, b, s, heads)
     assert torch.isfinite(ctx.float()).all()
     close(ctx.float(), ref, h16, 2.0)
+    # the packer refuses each of these rows on its own: identity layout, the padded result bit for bit
+    for bad in range(b):
+        m = torch.ones_like(mask)
+        m[:, 60:] = 0
+        m[bad] = mask[bad]
+        check_packed(qkv, m, nv.attention_d64(qkv, m, b, s, heads), None, None, h16, 2.0, heads=heads)
 
 
 def test_attention_many_items_per_cta(dev, h16, att_variant):
@@ -134,6 +251,7 @@ def test_attention_many_items_per_cta(dev, h16, att_variant):
     valid = mask.bool().view(-1)
     close(ctx.float()[valid], ref[valid], h16, 2.0)
     assert torch.isfinite(ctx.float()).all()
+    check_packed(qkv, mask, ctx, ref, valid, h16, 2.0, heads=heads)
 
 
 def test_attention_large_scores_trigger_rescale(dev, h16, att_variant):
@@ -148,6 +266,14 @@ def test_attention_large_scores_trigger_rescale(dev, h16, att_variant):
     mask = torch.ones(b, s, dtype=torch.int64, device=dev)
     ctx = nv.attention_d64(qkv, mask, b, s, heads)
     close(ctx.float(), ref_attention(qkv, mask, b, s, heads), h16, 3.0)
+    # the same ramp on the packed layout: the first sequence stops mid-chunk, its successor starts there
+    mask[0, 301:] = 0
+    mask[1, 450:] = 0
+    ctx = nv.attention_d64(qkv, mask, b, s, heads)
+    ref = ref_attention(qkv, mask, b, s, heads)
+    valid = mask.bool().view(-1)
+    close(ctx.float()[valid], ref[valid], h16, 3.0)
+    check_packed(qkv, mask, ctx, ref, valid, h16, 3.0, heads=heads)
 
 
 @pytest.mark.parametrize('h', [256, 768, 1024, 1280])
@@ -271,24 +397,29 @@ def test_gemm_without_bias(dev, h16):
 
 
 def ref_attention_causal(qkv, mask, b, s, heads, kv_heads, window):
+    """fp32 reference, one sequence at a time; (context, query rows that see at least one key)."""
     d = 128
-    q = qkv[:, :heads * d].float().view(b, s, heads, d).permute(0, 2, 1, 3)
-    k = qkv[:, heads * d:(heads + kv_heads) * d].float().view(b, s, kv_heads, d).permute(0, 2, 1, 3)
-    v = qkv[:, (heads + kv_heads) * d:].float().view(b, s, kv_heads, d).permute(0, 2, 1, 3)
-    k = k.repeat_interleave(heads // kv_heads, dim=1)
-    v = v.repeat_interleave(heads // kv_heads, dim=1)
     i = torch.arange(s, device=qkv.device)[:, None]
     j = torch.arange(s, device=qkv.device)[None, :]
-    vis = j <= i
+    causal = j <= i
     if window:
-        vis = vis & (i - j < window)
-    vis = vis[None, None] & (mask != 0)[:, None, None, :]
-    scores = (q @ k.transpose(-1, -2)) * d ** -0.5
-    p = torch.softmax(scores.masked_fill(~vis, float('-inf')), dim=-1)
-    alive = vis.any(-1)                      # [B,1,S]: query rows with at least one visible key
-    p = torch.nan_to_num(p, nan=0.0)
-    out = (p @ v).permute(0, 2, 1, 3).reshape(b * s, heads * d)
-    return out, alive.expand(b, heads, s)[:, 0].reshape(b * s)
+        causal = causal & (i - j < window)
+    out = torch.empty(b, s, heads * d, device=qkv.device)
+    alive = torch.empty(b, s, dtype=torch.bool, device=qkv.device)
+    for r in range(b):
+        x = qkv[r * s:(r + 1) * s].float()
+        q = x[:, :heads * d].view(s, heads, d).transpose(0, 1)
+        k = x[:, heads * d:(heads + kv_heads) * d].view(s, kv_heads, d).transpose(0, 1)
+        v = x[:, (heads + kv_heads) * d:].view(s, kv_heads, d).transpose(0, 1)
+        k = k.repeat_interleave(heads // kv_heads, dim=0)
+        v = v.repeat_interleave(heads // kv_heads, dim=0)
+        vis = causal & (mask[r] != 0)[None, :]
+        scores = ((q @ k.transpose(-1, -2)) * d ** -0.5).masked_fill_(~vis, float('-inf'))
+        p = torch.nan_to_num(torch.softmax(scores, dim=-1), nan=0.0)
+        del scores
+        out[r] = (p @ v).transpose(0, 1).reshape(s, heads * d)
+        alive[r] = vis.any(-1)
+    return out.view(b * s, heads * d), alive.view(b * s)
 
 
 CAUSAL_CASES = [
@@ -298,6 +429,9 @@ CAUSAL_CASES = [
     (1, 1100, 2, 1, 0, 'none'), (1, 1100, 2, 1, 300, 'left'), (4, 37, 2, 1, 16, 'right'),
     (5, 1, 2, 2, 0, 'none'), (2, 640, 8, 2, 128, 'none'), (2, 300, 4, 4, 1, 'none'),
     (2, 400, 2, 1, 64, 'right'), (2, 400, 2, 1, 65, 'left'),
+    # production lengths: Mistral-7B's S = 4096 without and with its window, positions far past the window
+    (2, 4096, 4, 1, 0, 'right'), (2, 4096, 2, 1, 4096, 'right'), (2, 8192, 2, 1, 4096, 'right'),
+    (2, 2049, 2, 1, 1000, 'left'),
 ]
 
 
@@ -318,6 +452,7 @@ def test_attention_causal_d128_matches_reference(dev, b, s, heads, kv_heads, win
     # rows that see no key at all (queries inside left padding) are unspecified; everything else,
     # including padded query positions that still see attended keys, must match
     close(ctx.float()[alive], ref[alive], h16, 2.0)
+    check_packed(qkv, mask, ctx, ref, alive, h16, 2.0, heads=heads, kv_heads=kv_heads, head_dim=128, window=window)
 
 
 def test_attention_causal_d128_many_items_and_rescale(dev, h16):
@@ -336,6 +471,7 @@ def test_attention_causal_d128_many_items_and_rescale(dev, h16):
     sel = alive & mask.bool().view(-1)
     assert torch.isfinite(ctx.float()).all()
     close(ctx.float()[sel], ref[sel], h16, 3.0)
+    check_packed(qkv, mask, ctx, ref, alive, h16, 3.0, heads=heads, kv_heads=kv_heads, head_dim=128, window=window)
 
 
 # ---------------------------------------------------------------------------- exact inner-product top-k
@@ -514,7 +650,7 @@ def test_gemm_geglu_epilogue(dev, m, i, k, h16):
 
 
 @pytest.mark.parametrize('b,s,heads,window', [(2, 512, 4, 64), (3, 333, 2, 64), (1, 1500, 2, 64), (2, 200, 4, 16),
-                                              (2, 700, 2, 300)])
+                                              (2, 700, 2, 300), (2, 8192, 2, 64)])
 def test_attention_d64_sliding_window(dev, b, s, heads, window, h16, att_variant):
     """Bidirectional sliding window |i - j| <= window (ModernBERT's local layers) on ragged batches; rows of
     padding tiles must stay finite."""
@@ -524,15 +660,11 @@ def test_attention_d64_sliding_window(dev, b, s, heads, window, h16, att_variant
     for r in range(1, b):
         mask[r, max(1, s - 90 * r):] = 0
     ctx = nv.attention_d64_window(qkv, mask, b, s, heads, window)
-    q, k, v = qkv.float().view(b, s, 3, heads, 64).unbind(2)
-    q, k, v = (t.permute(0, 2, 1, 3) for t in (q, k, v))
-    i = torch.arange(s, device=dev)
-    vis = ((i[:, None] - i[None, :]).abs() <= window)[None, None] & (mask != 0)[:, None, None, :]
-    scores = (q @ k.transpose(-1, -2) / 8.0).masked_fill(~vis, torch.finfo(torch.float32).min)
-    ref = (torch.softmax(scores, -1) @ v).permute(0, 2, 1, 3).reshape(b * s, heads * 64)
+    ref = ref_attention(qkv, mask, b, s, heads, window)
     valid = mask.bool().view(-1)
     assert torch.isfinite(ctx.float()).all()
     close(ctx.float()[valid], ref[valid], h16, 2.0)
+    check_packed(qkv, mask, ctx, ref, valid, h16, 2.0, heads=heads, window=window)
 
 
 # ------------------------------------------------------------------------- profiling instantiations
